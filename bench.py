@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps 4 --warmup 1      # CPU reference arm (oracle port)
+    python bench.py --steps 10 --warmup 3 --dump-outputs DIR   # + the results of the last timed step as DIR/*.npy
 
 --config selects the BASELINE.json configuration (SURVEY.md 8d); the default, 2, is the one the metric is quoted on:
   2  batch 32/GPU x 600x900, fp32-faithful conv arithmetic, DETECT_MODE H             (configs[1])
@@ -83,7 +84,12 @@ def parse():
     ap.add_argument("--alt-modes", type=int, default=1, help="config 2 on 1 GPU: also time the bf16x2 (3-unit) and bf16 (configs[2]) arithmetic")
     ap.add_argument("--cpu-sample", type=int, default=4, help="images in the cpu_baseline sample (0: skip that leg)")
     ap.add_argument("--connector-threads", type=int, default=8)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the timed path returned in its last step to DIR/*.npy (inputs are seeded: two builds compare file by file)")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 class ClockSampler:
@@ -259,6 +265,34 @@ def nms_vs_reference(eng, n=12000, reps=5):
     return res
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, packed, shapes, per_shape, rows, world):
+    """Results of one step as DIR/rois_<H>x<W>.npy (float32 [images, rows, 5] = score, x1, y1, x2, y2; rows past an image's
+    count are zero, as the engine returns them) and DIR/count_<H>x<W>.npy (float64 [images]), images in rank order.
+    Above DUMP_BYTES in all, a fixed seeded sample of the images of each shape is written, their indices in
+    DIR/image_index_<H>x<W>.npy."""
+    import numpy as np
+    import torch
+    flat = torch.cat([p.reshape(-1) for p in packed]).cpu().numpy().reshape(world, -1)
+    n_img = world * per_shape
+    keep = min(n_img, DUMP_BYTES // (len(shapes) * (rows * 5 * 4 + 8)))
+    os.makedirs(out_dir, exist_ok=True)
+    off = 0
+    for H, W in shapes:
+        n_rois = per_shape * rows * 5
+        rois = flat[:, off:off + n_rois].reshape(n_img, rows, 5)
+        count = np.ascontiguousarray(flat[:, off + n_rois:off + n_rois + per_shape]).view(np.int32).reshape(n_img)
+        off += n_rois + per_shape
+        if keep < n_img:
+            idx = np.sort(np.random.RandomState(0).choice(n_img, keep, replace=False))
+            rois, count = rois[idx], count[idx]
+            np.save(os.path.join(out_dir, "image_index_%dx%d.npy" % (H, W)), idx.astype(np.float64))
+        np.save(os.path.join(out_dir, "rois_%dx%d.npy" % (H, W)), np.ascontiguousarray(rois, dtype=np.float32))
+        np.save(os.path.join(out_dir, "count_%dx%d.npy" % (H, W)), count.astype(np.float64))
+
+
 def run_reference(a, cfg):
     """Reference arm: the reference's CPU path restated (oracle port; TF 1.3 cannot be installed),
     one image per step, all host threads."""
@@ -334,6 +368,7 @@ def main():
 
     gather_stream = torch.cuda.Stream(device=dev) if world > 1 else None
     inflight = []            # (packed, gathered, work) of every step of the current region: released only after the region
+    latest = []              # what the latest step returned (--dump-outputs)
 
     def step_device():
         outs = [eng.detect_packed(im, info) for im, info in zip(images, infos)]
@@ -350,6 +385,7 @@ def main():
                 work = dist.all_gather_into_tensor(gathered, packed, async_op=True)
             inflight.append((packed, gathered, work))
             outs = [gathered]
+        latest[:] = outs
         return outs
 
     def drain():
@@ -407,6 +443,7 @@ def main():
     e1.record()
     barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
+    timed_outs = list(latest)
     del inflight[:]
     if not prof_inside:
         N.check(N.lib.ctpn_prof_enable(1), "prof")
@@ -560,6 +597,8 @@ def main():
             line["parity"] = {"mode": mode, "vs": "float32 CPU oracle, one synthetic image per shape", "images": parity_vs_oracle(eng, shapes)}
             if a.config == 2:
                 line["nms_vs_reference"] = nms_vs_reference(eng)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, timed_outs, shapes, per_shape, post, world)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

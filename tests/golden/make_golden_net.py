@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Generate tests/golden/reference_net_wiring.npz by running the REFERENCE's own inference code -- get_network("VGGnet_test")
+"""Generate tests/golden/reference_net_wiring*.npz by running the REFERENCE's own inference code -- get_network("VGGnet_test")
 (lib/networks/factory.py, VGGnet_test.py, network.py), test_ctpn (lib/fast_rcnn/test.py) and, through tf.py_func, its
 proposal layer -- imported unmodified from /root/reference, on top of tests/golden/tf1_stub (a numpy stand-in for the few
 TensorFlow 1.x graph functions that code calls; TensorFlow 1.3 itself cannot be installed here).
@@ -10,6 +10,7 @@ Build container only:
     make -C oracle && python tests/golden/make_golden_net.py
 cfg.TEST.SCALES / MAX_SIZE are reduced so that the numpy convolutions finish in seconds and the fixture stays small; the
 weights are oracle/synth.py::make_weights(seed) keyed by the TF variable names."""
+import io
 import os
 import sys
 
@@ -27,6 +28,25 @@ CASES = [  # tag, weight seed, image seed, h, w, SCALES, MAX_SIZE
     ("capped_odd", 2, 13, 70, 190, 100, 150),     # MAX_SIZE cap; odd feature-map sizes (pool flooring)
 ]
 TAPS = ("conv1_1", "pool1", "conv5_3", "rpn_conv/3x3", "lstm_o", "rpn_cls_score", "rpn_bbox_pred", "rpn_cls_prob_reshape")
+PART_BYTES = 1000000      # every fixture file stays below 1 MB: reference_net_wiring.npz, reference_net_wiring_2.npz, ...
+
+
+def save_parts(out):
+    """np.savez_compressed of `out` in key order, starting the next file before one would reach PART_BYTES."""
+    parts, part = [], {}
+    for k, v in out.items():
+        part[k] = v
+        buf = io.BytesIO()
+        np.savez_compressed(buf, **part)
+        if buf.tell() >= PART_BYTES and len(part) > 1:
+            del part[k]
+            parts.append(part)
+            part = {k: v}
+    parts.append(part)
+    for i, arrays in enumerate(parts):
+        path = os.path.join(HERE, "reference_net_wiring%s.npz" % ("_%d" % (i + 1) if i else ""))
+        np.savez_compressed(path, **arrays)
+        print("wrote", path, os.path.getsize(path), "bytes")
 
 
 def main():
@@ -66,9 +86,7 @@ def main():
             out["%s_%s" % (tag, name.replace("/", "_"))] = val.astype(np.float32)
         print(tag, "blob", blobs["data"].shape, "scale %.4f" % im_scales[0], "rois", scores.shape[0],
               "heads", taps[TAPS.index("rpn_cls_score")].shape)
-    path = os.path.join(HERE, "reference_net_wiring.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path), "bytes")
+    save_parts(out)
 
 
 if __name__ == "__main__":

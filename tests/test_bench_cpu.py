@@ -58,3 +58,28 @@ def test_committed_bench_lines_parse_and_name_their_configuration():
         seen.add((d["config"]["baseline_config"], d["n_gpus"]))
     assert {c for c, _n in seen} >= {"BASELINE.json configs[%d] (--config %d)" % (i - 1, i) for i in (2, 3, 4, 5)}
     assert {n for _c, n in seen} >= {1, 4, 8}
+
+
+def test_dump_outputs_unpacks_rank_and_shape_buckets(tmp_path, monkeypatch):
+    """--dump-outputs: the packed step results (per rank: each shape bucket's rois, then its int32 counts) come out as one
+    rois / count pair per shape, images in rank order; above the byte cap a fixed sample of the images is written."""
+    import numpy as np
+    import torch
+    shapes, per_shape, rows, world = [(600, 900), (900, 600)], 2, 3, 2
+    rois = np.arange(world * len(shapes) * per_shape * rows * 5, dtype=np.float32).reshape(world, len(shapes), per_shape, rows, 5)
+    count = np.arange(world * len(shapes) * per_shape, dtype=np.int32).reshape(world, len(shapes), per_shape)
+    packed = torch.from_numpy(np.concatenate([np.concatenate([rois[r, s].reshape(-1), count[r, s].view(np.float32)])
+                                              for r in range(world) for s in range(len(shapes))]))
+    bench.dump_outputs(str(tmp_path / "a"), [packed], shapes, per_shape, rows, world)
+    for s, (H, W) in enumerate(shapes):
+        got = np.load(tmp_path / "a" / ("rois_%dx%d.npy" % (H, W)))
+        assert got.dtype == np.float32 and np.array_equal(got, rois[:, s].reshape(world * per_shape, rows, 5))
+        got = np.load(tmp_path / "a" / ("count_%dx%d.npy" % (H, W)))
+        assert got.dtype == np.float64 and np.array_equal(got, count[:, s].reshape(-1))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2 * (rows * 5 * 4 + 8) * len(shapes))
+    bench.dump_outputs(str(tmp_path / "b"), [packed], shapes, per_shape, rows, world)
+    for s, (H, W) in enumerate(shapes):
+        idx = np.load(tmp_path / "b" / ("image_index_%dx%d.npy" % (H, W))).astype(int)
+        assert len(idx) == 2 and np.array_equal(idx, np.unique(idx))
+        got = np.load(tmp_path / "b" / ("rois_%dx%d.npy" % (H, W)))
+        assert np.array_equal(got, rois[:, s].reshape(world * per_shape, rows, 5)[idx])

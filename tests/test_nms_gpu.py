@@ -1,6 +1,7 @@
 """GPU: NMS through the C ABI (ctpn_nms_host via the reference-named wrappers nms()/gpu_nms())
 is bit-exact against the CPU oracle and the reference-generated golden keep lists."""
 import ctypes as C
+import hashlib
 import os
 
 import numpy as np
@@ -11,6 +12,7 @@ from oracle import postproc, synth
 pytestmark = pytest.mark.gpu
 G = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_postproc.npz"))
 NMS_TAGS = sorted(k[4:-5] for k in G.files if k.startswith("nms_") and k.endswith("_keep"))
+REF_KERNEL = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_nms_kernel.npz"))
 
 
 @pytest.mark.parametrize("tag", NMS_TAGS)
@@ -73,31 +75,20 @@ def test_nms_sorted_batched_early_exit():
     assert rc == 3 and "workspace" in N.last_error()
 
 
-def _load_reference_nms():
-    """The reference's own CUDA NMS (lib/utils/nms_kernel.cu) built by oracle/Makefile into oracle/_ref/."""
-    import ctypes
-    path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libref_nms.so")
-    if not os.path.exists(path):
-        pytest.skip("oracle/_ref/libref_nms.so not built (needs /root/reference at build time)")
-    lib = ctypes.CDLL(path)
-    lib.ref_nms.restype = None
-    lib.ref_nms.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_int]
-    return lib
-
-
 @pytest.mark.parametrize("n,thresh,ctpn_like", [(3000, 0.7, False), (6000, 0.7, True), (2000, 0.2, True)])
 def test_against_the_reference_cuda_kernel(n, thresh, ctpn_like):
-    """ctpn_nms_host vs the reference's `_nms` on identical sorted boxes.  The reference kernel is compiled with nvcc's
+    """ctpn_nms_host vs the reference's `_nms` on identical sorted boxes, through the keep lists that kernel produced on a
+    B200 (tests/golden/make_golden_nms.py -> reference_nms_kernel.npz).  The reference kernel is compiled with nvcc's
     default FMA contraction, so an IoU within 1 ulp of the threshold may decide differently; everything else must agree."""
-    ref = _load_reference_nms()
     from ctpn_b200 import _native as N
+    tag = "n%d_t%g_%s" % (n, thresh, "ctpn" if ctpn_like else "generic")
     dets = synth.make_boxes(77 + n % 5, n, ctpn_like=ctpn_like)
     dets = np.ascontiguousarray(dets[postproc.order_desc(dets[:, 4])])
-    keep_r = np.zeros(n, np.int32); num_r = C.c_int(0)
-    ref.ref_nms(keep_r.ctypes.data, C.byref(num_r), dets.ctypes.data, n, 5, np.float32(thresh), 0)
+    assert hashlib.sha256(dets.tobytes()).hexdigest() == str(REF_KERNEL[tag + "_boxes_sha256"]), \
+        "the boxes differ from those the stored keep list was computed on"
     keep_o = np.zeros(n, np.int32); num_o = C.c_int(0)
     N.check(N.lib.ctpn_nms_host(keep_o.ctypes.data, C.byref(num_o), dets.ctypes.data, n, 5, np.float32(thresh), 0), "ctpn_nms_host")
-    a, b = keep_r[:num_r.value].tolist(), keep_o[:num_o.value].tolist()
+    a, b = REF_KERNEL[tag + "_keep"].tolist(), keep_o[:num_o.value].tolist()
     np.testing.assert_array_equal(np.asarray(b), postproc.nms_sorted(dets, thresh))      # ours == CPU oracle, always
     if a != b:
         sa, sb = set(a), set(b)

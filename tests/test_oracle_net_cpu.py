@@ -38,18 +38,22 @@ def test_restatements_agree_on_a_batch_and_reverse_direction_matters():
 
 
 # ---- the oracle against the reference's OWN graph code ---------------------------------------------------------------------
-# tests/golden/reference_net_wiring.npz: get_network("VGGnet_test") + test_ctpn + the py_func proposal layer, imported
+# tests/golden/reference_net_wiring*.npz: get_network("VGGnet_test") + test_ctpn + the py_func proposal layer, imported
 # unmodified from /root/reference and executed on tests/golden/tf1_stub (numpy stand-ins for the TensorFlow functions that
 # code calls).  Pins the wiring (layer order, variable names, row sequences, fw/bw concatenation, reshapes, pair softmax,
 # blob / im_info handling); the per-op semantics inside the stub are a restatement, like the oracle's.
+import glob  # noqa: E402
 import os  # noqa: E402
 
 import pytest  # noqa: E402
 
 from oracle import postproc  # noqa: E402
 
-WIRING = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_net_wiring.npz"))
-WIRING_TAGS = sorted(k[:-4] for k in WIRING.files if k.endswith("_cfg"))
+WIRING = {}
+for _part in sorted(glob.glob(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_net_wiring*.npz"))):
+    with np.load(_part) as _z:          # one fixture, split over files of less than 1 MB each (make_golden_net.py)
+        WIRING.update(_z)
+WIRING_TAGS = sorted(k[:-4] for k in WIRING if k.endswith("_cfg"))
 
 
 def test_reference_graph_asks_for_exactly_the_variables_the_engine_requires():
